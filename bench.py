@@ -5,6 +5,7 @@ per-cell count).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
   python bench.py --impl reference [--steps K] [--warmup W]      # the reference algorithm on the host CPU
+  python bench.py --gpus 1 [...] --dump-outputs DIR               # also write the last timed step's outputs (dump_outputs)
 
 Workload (BASELINE.json configs[3], the one the metric is quoted on): 2-D thermal convection,
 Ra=1e6, Arrhenius viscosity clipped to [1e17,1e23], 4096^2 cells (4097^2 nodes), 16 markers/cell
@@ -183,6 +184,8 @@ def run_b200(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs one GPU (on several the markers and grid rows are split over the ranks)")
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -254,6 +257,8 @@ def run_b200(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = float(t.item()) / args.steps
+    if args.dump_outputs:                        # before the e2e leg moves the state on
+        dump_outputs(s, args.per_side, args.dump_outputs)
 
     # ---- e2e: the same step through host buffers (rank-local) ----
     e2e = None
@@ -344,6 +349,51 @@ def run_b200(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_NODES, DUMP_MARKERS, DUMP_SEED, DUMP_MAX_BYTES = 1 << 19, 1 << 18, 2024, 64 * 10 ** 6
+
+
+def dump_outputs(s, per_side, out_dir):
+    """Writes what the last timed step hands back, the arrays of the reference's per-step output (pylamp2.py:637-650,
+    driver.save_npz): the grids velz, velx, pres, rho, temp and the markers' tr_x (M,2), tr_f (M,13), tr_v (M,2), as
+    out_dir/<name>.npy in float64.  A fixed seeded sample keeps the files under DUMP_MAX_BYTES: DUMP_NODES nodes of
+    every grid (flat indices, ascending) and every marker of DUMP_MARKERS / per_side^2 cells, ordered by (cell, z, x)
+    -- the device sort orders the markers of one cell by the arrival of its atomics, so the sample is put in an order
+    of its own that two runs of one build share.  The cells are those the markers sit in after the last step, and the
+    markers carry no identity (the TR__ID column of this workload is zero): where two builds move a marker to
+    different sides of a sampled cell's edge, the marker arrays differ in length or shift by a row, so compare two
+    builds' markers cell by cell (the cell of a row follows from its tr_x), not row by row.  The grid samples always
+    align."""
+    import torch
+    nz, nxx = s.nx
+    dev = s.tr_x.device
+    rng = np.random.default_rng(DUMP_SEED)
+    nodes = np.sort(rng.choice(nz * nxx, min(nz * nxx, DUMP_NODES), replace=False))
+    ncells = (nz - 1) * (nxx - 1)
+    cells = rng.choice(ncells, min(ncells, max(1, DUMP_MARKERS // per_side ** 2)), replace=False)
+    inode = torch.as_tensor(nodes, device=dev)
+    out = {name: f.reshape(-1)[inode].cpu().numpy() for name, f in
+           (("velz", s.newvel[0]), ("velx", s.newvel[1]), ("pres", s.newpres), ("rho", s.f_rho), ("temp", s.newtemp))}
+    # cell of every marker: floor((n-1)*x/L) clamped into the box, the key of the device sort
+    ie = torch.floor((nz - 1) * s.tr_x[:, 0] / s.L[0]).clamp_(0, nz - 2).long()
+    key = ie * (nxx - 1) + torch.floor((nxx - 1) * s.tr_x[:, 1] / s.L[1]).clamp_(0, nxx - 2).long()
+    del ie
+    picked = torch.zeros(ncells, dtype=torch.bool, device=dev)
+    picked[torch.as_tensor(cells, device=dev)] = True
+    m = torch.nonzero(picked[key]).squeeze(1)
+    key = key[m].cpu().numpy()
+    x = s.tr_x[m].cpu().numpy()
+    m = m[torch.as_tensor(np.lexsort((x[:, 1], x[:, 0], key)), device=dev)]
+    out["tr_x"] = s.tr_x[m].cpu().numpy()
+    out["tr_f"] = torch.stack([c[m] for c in s.cols], dim=1).cpu().numpy()
+    out["tr_v"] = s.trac_vel[m].cpu().numpy()
+    nbytes = sum(a.nbytes for a in out.values())
+    if nbytes > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (nbytes, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_e2e(torch, driver, s, o, nsteps):
     """The same timestep through HOST buffers.  What a time step takes in and hands back is the state that changes:
     marker coordinates and marker temperature go from pinned host memory to the device, the step runs, and the new
@@ -432,7 +482,13 @@ def main():
     ap.add_argument("--seed", type=int, default=11, help="seed of the marker jitter (rank r uses seed + 1000 r)")
     ap.add_argument("--cpu-ncell", type=int, default=256, help="CPU-baseline sample size (0 = skip)")
     ap.add_argument("--ref-ncell", type=int, default=256, help="--impl reference sample size")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write a fixed sample of what the last one computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

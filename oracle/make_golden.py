@@ -3,7 +3,7 @@
     python oracle/make_golden.py
 
 The reference ships no golden vectors (SURVEY.md §4); these are outputs of the reference
-modules themselves (imported from /root/reference through oracle/ref_shims.py) on seeded
+modules themselves (imported through oracle/ref_shims.py from PYLAMP_REFERENCE_DIR) on seeded
 inputs.  The inputs are stored next to the outputs so the tests never need the reference.
 Test infrastructure only.
 """

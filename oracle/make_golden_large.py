@@ -1,10 +1,10 @@
-"""Solver-parity fixtures at sizes where one direct solve costs minutes to half an hour (build
-container only; run once, results committed as strided samples under tests/golden/large_*.npz).
+"""Solver-parity fixtures at sizes where one direct solve costs minutes to half an hour (needs the original
+PyLamp; run once, results committed as strided samples under tests/golden/large_*_0.npz, _1.npz).
 
     python oracle/make_golden_large.py conv513 solcx513 conv1025 solcx1025
 
 For every case the UNMODIFIED reference assembles the system (pylamp_stokes.makeStokesMatrix,
-imported from /root/reference through oracle/ref_shims.py) and SciPy's SuperLU solves it the way
+imported through oracle/ref_shims.py from PYLAMP_REFERENCE_DIR) and SciPy's SuperLU solves it the way
 pylamp2.py:360 does; one fp64 refinement step on top is the ground truth (SURVEY.md 8c).  The inputs
 are analytic (pylamp_b200/setups.py: `convection_fields(ncell, t=0)`, `solcx_fields(n)`), so only
 the solution has to be stored: every `stride`-th node in both directions (257 x 257 samples) of vz,
@@ -22,9 +22,9 @@ import scipy.sparse.linalg
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import ref_shims  # noqa: E402
+from oracle.large_fixtures import save  # noqa: E402
 from pylamp_b200 import setups  # noqa: E402
 
-OUT = os.path.join(ROOT, "tests", "golden")
 CASES = {"conv513": ("conv", 512), "conv1025": ("conv", 1024), "solcx513": ("solcx", 512),
          "solcx1025": ("solcx", 1024), "conv257": ("conv", 256), "solcx257": ("solcx", 256)}
 
@@ -62,7 +62,7 @@ def make(name):
         full, raw = x[k::3], x_raw[k::3]
         out[nm + "_norm"] = np.linalg.norm(full)
         out[nm + "_floor"] = np.linalg.norm(raw - full) / np.linalg.norm(full)   # raw spsolve <-> refined, all nodes
-    np.savez_compressed(os.path.join(OUT, "large_%s.npz" % name), **out)
+    save(name, out)
     print(name, "nx", nx, "assemble %.1f s, splu+solve %.1f s" % (t_asm, t_solve), "residual raw %.2e refined %.2e" %
           (res_raw, res_ref), "floor", [float("%.2e" % out[n + "_floor"]) for n in ("vz", "vx", "p")], flush=True)
 

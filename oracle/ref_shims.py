@@ -1,8 +1,10 @@
-"""Import the UNMODIFIED reference from /root/reference -- test infrastructure only.
+"""Import the UNMODIFIED reference -- test infrastructure only.
 
-Only usable in the build container (``/root/reference`` does not exist on the GPU
-box).  Used by ``oracle/make_golden.py`` to generate ``tests/golden/*.npz`` and by
-``tests/test_oracle_vs_reference.py`` (skipped when the reference is absent).
+Only usable where the environment variable ``PYLAMP_REFERENCE_DIR`` names a checkout of the
+original PyLamp (the repository does not contain it).  Used by ``oracle/make_golden.py`` and
+``oracle/make_golden_large.py`` to generate ``tests/golden/*.npz``, and by
+``tests/test_reference_bc_probe.py`` and ``tests/test_launcher_gpu.py``, which skip when the
+reference is absent.
 
 Three non-invasive shims (SURVEY.md Appendix A), none of which touches a reference file:
   1. ``pylamp_trac`` passes a *list* as a multi-axis index to ``np.add.at``
@@ -19,11 +21,11 @@ import types
 
 import numpy as _np
 
-REFERENCE_DIR = os.environ.get("PYLAMP_REFERENCE_DIR", "/root/reference")
+REFERENCE_DIR = os.environ.get("PYLAMP_REFERENCE_DIR", "")
 
 
 def available():
-    return os.path.isfile(os.path.join(REFERENCE_DIR, "pylamp_trac.py"))
+    return bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "pylamp_trac.py"))
 
 
 class _Add:

@@ -5,7 +5,7 @@
 Steps the analytic C4-type fields (setups.convection_fields) through t = -nsteps..0 with the time-loop
 solver settings of bench.py (warm start by extrapolation, eigenvalue estimates every 8 steps), then
   (a) for every rtol given: re-runs the sequence and reports iterations / relres / status of the last solve
-      and, when tests/golden/large_conv<ncell+1>.npz exists, its error against the reference's direct solve;
+      and, when the fixture tests/golden/large_conv<ncell+1>_*.npz exists, its error against the reference's direct solve;
   (b) one cold solve at rtol 1e-14 with PLB_DEBUG_FGMRES=1 to show the true-residual history (the fp64 floor).
 """
 import os
@@ -18,13 +18,16 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
+from oracle import large_fixtures  # noqa: E402
 from pylamp_b200 import pylamp_stokes as S, setups  # noqa: E402
 
 ncell = int(sys.argv[1])
 nsteps = int(sys.argv[2]) if len(sys.argv) > 2 else 12
 rtols = [float(v) for v in sys.argv[3:]] or [1e-9, 1e-10, 1e-11, 1e-12]
-fx = os.path.join(ROOT, "tests", "golden", "large_conv%d.npz" % (ncell + 1))
-gold = np.load(fx) if os.path.exists(fx) else None
+try:
+    gold = large_fixtures.load("conv%d" % (ncell + 1))
+except FileNotFoundError:
+    gold = None
 dev = torch.device("cuda")
 
 

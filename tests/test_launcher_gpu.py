@@ -1,18 +1,20 @@
-"""INTEGRATION.md 3: the UNMODIFIED reference driver /root/reference/pylamp2.py executed on top of the
+"""INTEGRATION.md 3: the UNMODIFIED reference driver pylamp2.py executed on top of the
 drop-in modules (pylamp_b200.launcher: module registration + the spsolve/csc_matrix rebinding), and its
 np.savez payload compared with the golden dump of the same script run on the reference's own modules
-(tests/golden/c1_noinject.npz, oracle/make_golden.py).  The reference checkout only exists in the build
-container; on a box without it the test is skipped (nothing can stand in for the reference's script)."""
+(tests/golden/c1_noinject.npz, oracle/make_golden.py).  The script is the original PyLamp's and not part of this
+repository: the test runs where PYLAMP_REFERENCE_DIR names a checkout of it and is skipped elsewhere (nothing can
+stand in for the reference's script)."""
 import os
 
 import numpy as np
 import pytest
 
 from conftest import GOLDEN
+from oracle.ref_shims import REFERENCE_DIR as REF
 
-REF = os.environ.get("PYLAMP_REFERENCE_DIR", "/root/reference")
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "pylamp2.py")), reason="reference checkout absent")]
+              pytest.mark.skipif(not (REF and os.path.isfile(os.path.join(REF, "pylamp2.py"))),
+                                 reason="needs a checkout of the original PyLamp in PYLAMP_REFERENCE_DIR")]
 
 
 def test_unmodified_pylamp2_on_dropin_modules_matches_golden():

@@ -1,6 +1,6 @@
 """Which wall types of the reference's Stokes assembly (pylamp_stokes.py:177-189, :257-276, :303-321, :525-551)
 have a solution a drop-in can be held to (SURVEY.md §8f-4).  The probe runs the unmodified reference (only where
-/root/reference is mounted, i.e. in the build container):
+PYLAMP_REFERENCE_DIR names a checkout of the original PyLamp):
   * FLOWTHRU|FREESLIP (= 5) on the x = 0 wall: a REGULAR system (the anchor moves to cell (nz/2, 0)) -- supported by
     the drop-in since round 2 (tests/test_flowthru_gpu.py; round 1 had wrongly lumped it with the singular ones);
   * 5 on the x = L wall: the anchor lands on the ghost pressure column, the constant pressure stays undetermined
@@ -14,7 +14,7 @@ import pytest
 
 from oracle import ref_shims
 
-pytestmark = pytest.mark.skipif(not ref_shims.available(), reason="needs the reference checkout")
+pytestmark = pytest.mark.skipif(not ref_shims.available(), reason="needs a checkout of the original PyLamp in PYLAMP_REFERENCE_DIR")
 
 FREESLIP, NOSLIP, CYCLIC, FLOWTHRU = 1, 0, 2, 4
 

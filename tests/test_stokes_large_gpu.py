@@ -10,22 +10,13 @@ sequence of slowly translating fields ending at the fixture's t = 0 -- what cons
 to the solver -- and must match vz, vx and P~ to 1e-8 relative L2 (north_star), or 3x the reference's own
 raw-spsolve noise floor where that is larger (SolCx pressure: 1e-6..1e-5, SURVEY App. B).
 """
-import os
-
 import numpy as np
 import pytest
 
-from conftest import GOLDEN
+from oracle.large_fixtures import load as _load
 
 pytestmark = [pytest.mark.gpu]
 NSTEPS = 12      # > warm_start history (5) and > lmax_every (8): stale eigenvalue estimates are exercised
-
-
-def _load(name):
-    p = os.path.join(GOLDEN, "large_%s.npz" % name)
-    if not os.path.exists(p):
-        pytest.skip("fixture %s not generated (oracle/make_golden_large.py)" % name)
-    return np.load(p)
 
 
 def _errors(x, nx, g):
