@@ -127,7 +127,15 @@ int plb_migrate_plan(plb_ctx* ctx, long long M, const double* d_tr_x, int nz, do
 int plb_migrate_apply(plb_ctx* ctx, long long M, int narr, double* const* h_arrs, const int* h_width,
                       long long capacity_rows, int nz, double Lz, int c0, int c1, long long* h_M_new);
 int plb_halo_rows(plb_ctx* ctx, int narr, double* const* h_ptrs, const long long* h_row_doubles, int i0, int i1, int h);
+/* Snapshot writer (pylamp_b200/output.py): move `count` doubles from rank `src` to rank 0 -- ncclSend on rank src,
+ * ncclRecv into d_buf on rank 0, nothing on the other ranks or when src == 0 -- on the context's stream. */
+int plb_comm_to_root(plb_ctx* ctx, int src, double* d_buf, long long count);
 void plb_comm_destroy(plb_ctx* ctx);
+
+/* ---- snapshot output: pylamp2.py:637-650 writes tr_f as one row-major (M,13) array --------------------------
+ * Rows [r0, r0+n) of ncol <= 16 fp64 columns (SoA; columns may alias each other) -> the row-major (n, ncol) block
+ * d_out (which must not overlap a column).  n = 0 is a no-op.  Profiled as class 11, 16*ncol bytes per row. */
+int plb_pack_columns(plb_ctx* ctx, long long r0, long long n, int ncol, const double* const* h_cols, double* d_out);
 
 /* ---- the marker->grid targets of one time step in ONE pass over the markers -------------------
  * (pylamp2.py:309-313 calls trac2grid four times -- nodes, cell centres, the two half-staggered grids --

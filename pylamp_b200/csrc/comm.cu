@@ -246,6 +246,23 @@ int plb_allreduce(plb_ctx* ctx, double* d_buf, long long count, int op) {
     return plb_comm_allreduce(ctx, d_buf, (size_t)count, op);
 }
 
+// point-to-point move of `count` doubles from rank `src` to rank 0 on the context's stream (snapshot writer):
+// rank src sends d_buf, rank 0 receives into d_buf, every other rank (and src == 0) does nothing
+int plb_comm_to_root(plb_ctx* ctx, int src, double* d_buf, long long count) {
+    if (!ctx) return 1;
+    plb_comm* c = ctx->comm;
+    const int size = c ? c->size : 1;
+    if (src < 0 || src >= size || count < 0) PLB_FAIL(ctx, "plb_comm_to_root: src %d of %d ranks, count %lld", src, size, count);
+    if (size == 1 || src == 0 || count == 0 || (c->rank != src && c->rank != 0)) return 0;
+    if (!d_buf) PLB_FAIL(ctx, "plb_comm_to_root: null buffer");
+    PLB_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (c->rank == src)
+        PLB_NCCL(ctx, api.Send(d_buf, (size_t)count, NCCL_DOUBLE, 0, c->comm, ctx->stream));
+    else
+        PLB_NCCL(ctx, api.Recv(d_buf, (size_t)count, NCCL_DOUBLE, src, c->comm, ctx->stream));
+    return 0;
+}
+
 void plb_comm_destroy(plb_ctx* ctx) {
     if (!ctx || !ctx->comm) return;
     if (ctx->comm->comm) api.CommDestroy(ctx->comm->comm);

@@ -388,10 +388,7 @@ def timestep(s, o, want_kelem=True, phases=False):
 def save_npz(s, prefix, it=None):
     """Write the two per-step `.npz` files of the reference with its exact keys (pylamp2.py:637-650:
     `griddata.<it>.npz` = gridz, gridx, velz, velx, pres, rho, temp, tstep, time; `tracs.<it>.npz` =
-    tr_x, tr_f, tr_v), so that the reference's pylamp_post.py reads them unchanged (SURVEY.md 8f-2)."""
-    it = s.it if it is None else it
-    host = lambda t: t.detach().cpu().numpy() if t is not None else np.zeros(tuple(s.nx))
-    np.savez("%sgriddata.%d.npz" % (prefix, it), gridz=s.grid[IZ], gridx=s.grid[IX], velz=host(s.newvel[IZ]),
-             velx=host(s.newvel[IX]), pres=host(s.newpres), rho=host(s.f_rho), temp=host(s.newtemp),
-             tstep=it, time=s.totaltime)
-    np.savez("%stracs.%d.npz" % (prefix, it), tr_x=host(s.tr_x), tr_f=s.tr_f_host(), tr_v=host(s.trac_vel))
+    tr_x, tr_f, tr_v), so that the reference's pylamp_post.py reads them unchanged (SURVEY.md 8f-2).  On several
+    ranks a collective call: rank 0 writes the whole state of every rank (output.write_snapshot)."""
+    from .output import write_snapshot
+    write_snapshot(s, prefix, it)
