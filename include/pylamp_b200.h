@@ -130,12 +130,26 @@ int plb_halo_rows(plb_ctx* ctx, int narr, double* const* h_ptrs, const long long
 /* Snapshot writer (pylamp_b200/output.py): move `count` doubles from rank `src` to rank 0 -- ncclSend on rank src,
  * ncclRecv into d_buf on rank 0, nothing on the other ranks or when src == 0 -- on the context's stream. */
 int plb_comm_to_root(plb_ctx* ctx, int src, double* d_buf, long long count);
+/* Snapshot reader: in-place ncclBroadcast of `count` doubles of d_buf from rank 0 to every rank on the context's
+ * stream; nothing on one rank. */
+int plb_comm_from_root(plb_ctx* ctx, double* d_buf, long long count);
 void plb_comm_destroy(plb_ctx* ctx);
 
 /* ---- snapshot output: pylamp2.py:637-650 writes tr_f as one row-major (M,13) array --------------------------
  * Rows [r0, r0+n) of ncol <= 16 fp64 columns (SoA; columns may alias each other) -> the row-major (n, ncol) block
  * d_out (which must not overlap a column).  n = 0 is a no-op.  Profiled as class 11, 16*ncol bytes per row. */
 int plb_pack_columns(plb_ctx* ctx, long long r0, long long n, int ncol, const double* const* h_cols, double* d_out);
+/* Snapshot reader, the reverse: of a chunk of n file rows -- d_x (n,2), d_f (n,ncol <= 16) and optionally d_v (n,2),
+ * row-major, d_x 16-byte aligned -- the rows i in [r0, r1) whose cell row floor((nz-1)*z/Lz), clamped to [0, nz-2] (the migration's
+ * rule), lies in [c0, c1) are appended in chunk order at row `base` of d_tr_x (rows of 2), the ncol columns h_cols
+ * and, with d_v, d_trac_vel (rows of 2); base + selected rows must not exceed cap_rows.  d_tr_x == NULL: count only
+ * (d_f may be NULL).  Synchronises once; *h_count = rows selected.  A row of the chunk with a non-finite z is an
+ * error (nothing is written).  Profiled as class 11: 16 B per row counted, 8 * (2 + ncol + 2) B per row read and
+ * per row written. */
+int plb_unpack_rows(plb_ctx* ctx, long long n, const double* d_x, const double* d_f, int ncol, const double* d_v, int nz,
+                    double Lz, int c0, int c1, long long r0, long long r1, long long base, long long cap_rows,
+                    double* d_tr_x,
+                    double* const* h_cols, double* d_trac_vel, long long* h_count);
 
 /* ---- the marker->grid targets of one time step in ONE pass over the markers -------------------
  * (pylamp2.py:309-313 calls trac2grid four times -- nodes, cell centres, the two half-staggered grids --

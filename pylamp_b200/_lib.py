@@ -36,6 +36,8 @@ _PROTOS = {
     "plb_comm_destroy": (None, [VP]),
     "plb_comm_to_root": (I, [VP, I, VP, LL]),
     "plb_pack_columns": (I, [VP, LL, LL, I, PP, VP]),
+    "plb_comm_from_root": (I, [VP, VP, LL]),
+    "plb_unpack_rows": (I, [VP, LL, VP, VP, I, VP, I, D, I, I, LL, LL, LL, LL, VP, PP, VP, C.POINTER(LL)]),
     "plb_ctx_set_slab": (I, [VP, I, I, I]),
     "plb_inject_plan": (I, [VP, LL, VP, I, I, LL, LL, C.POINTER(LL)]),
     "plb_inject_apply": (I, [VP, LL, VP, VP, VP, I, PP, I, D, VP, VP, I, C.c_ulonglong, C.c_ulonglong]),

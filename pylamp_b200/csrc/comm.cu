@@ -24,6 +24,7 @@ struct NcclApi {
     int (*AllReduce)(const void*, void*, size_t, int, int, nccl_comm_t, cudaStream_t) = nullptr;
     int (*Send)(const void*, size_t, int, int, nccl_comm_t, cudaStream_t) = nullptr;
     int (*Recv)(void*, size_t, int, int, nccl_comm_t, cudaStream_t) = nullptr;
+    int (*Broadcast)(const void*, void*, size_t, int, int, nccl_comm_t, cudaStream_t) = nullptr;
     int (*GroupStart)() = nullptr;
     int (*GroupEnd)() = nullptr;
     const char* (*GetErrorString)(int) = nullptr;
@@ -46,6 +47,7 @@ int load_api(plb_ctx* ctx) {
     SYM(AllReduce, "ncclAllReduce");
     SYM(Send, "ncclSend");
     SYM(Recv, "ncclRecv");
+    SYM(Broadcast, "ncclBroadcast");
     SYM(GroupStart, "ncclGroupStart");
     SYM(GroupEnd, "ncclGroupEnd");
     SYM(GetErrorString, "ncclGetErrorString");
@@ -260,6 +262,19 @@ int plb_comm_to_root(plb_ctx* ctx, int src, double* d_buf, long long count) {
         PLB_NCCL(ctx, api.Send(d_buf, (size_t)count, NCCL_DOUBLE, 0, c->comm, ctx->stream));
     else
         PLB_NCCL(ctx, api.Recv(d_buf, (size_t)count, NCCL_DOUBLE, src, c->comm, ctx->stream));
+    return 0;
+}
+
+// in-place broadcast of `count` doubles from rank 0 to every rank on the context's stream (snapshot reader);
+// nothing on one rank
+int plb_comm_from_root(plb_ctx* ctx, double* d_buf, long long count) {
+    if (!ctx) return 1;
+    plb_comm* c = ctx->comm;
+    if (count < 0) PLB_FAIL(ctx, "plb_comm_from_root: count %lld", count);
+    if (!c || c->size == 1 || count == 0) return 0;
+    if (!d_buf) PLB_FAIL(ctx, "plb_comm_from_root: null buffer");
+    PLB_CUDA(ctx, cudaSetDevice(ctx->device));
+    PLB_NCCL(ctx, api.Broadcast(d_buf, d_buf, (size_t)count, NCCL_DOUBLE, 0, c->comm, ctx->stream));
     return 0;
 }
 

@@ -12,6 +12,7 @@
 // All marker kernels are order-independent, so which slot a marker lands in does not matter.
 #include <vector>
 
+#include "cell_row.cuh"
 #include "comm.cuh"
 
 struct plb_migrate_ws {
@@ -28,11 +29,6 @@ struct plb_migrate_ws {
 };
 
 namespace {
-
-__device__ __forceinline__ int row_of(double z, int nz, double Lz) {
-    long long ie = (long long)floor(__ddiv_rn(__dmul_rn((double)(nz - 1), z), Lz));
-    return ie < 0 ? 0 : (ie > nz - 2 ? nz - 2 : (int)ie);
-}
 
 __global__ void __launch_bounds__(256)
 k_mig_list(long long M, const double2* __restrict__ trx, int nz, double Lz, int c0, int c1, int lo_ok, int hi_ok,

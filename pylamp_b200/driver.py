@@ -11,7 +11,7 @@ markers (SoA columns) and grid fields on the GPU and is what `bench.py` times.
 
 Mirrors oracle/pylamp_oracle.py's State/Options/timestep so that the parity tests read the same on
 both sides.  Marker injection (`tracdens_min > 0`), marker removal (`tracs_fence_enabled=False`) and the
-`.npz` output (`save_npz`) are the SURVEY.md §8f rows built so far.
+`.npz` output (`save_npz`, read back by `load_npz`) are the SURVEY.md §8f rows built so far.
 """
 import numpy as np
 import torch
@@ -392,3 +392,11 @@ def save_npz(s, prefix, it=None):
     ranks a collective call: rank 0 writes the whole state of every rank (output.write_snapshot)."""
     from .output import write_snapshot
     write_snapshot(s, prefix, it)
+
+
+def load_npz(prefix, it, o, device=None):
+    """The state of a `save_npz` pair (or of the reference's own `griddata.<it>.npz` / `tracs.<it>.npz`), ready for
+    `timestep(s, o)`: a collective call on several ranks, where `o.marker_ownership` decides which markers each rank
+    keeps (output.read_snapshot)."""
+    from .output import read_snapshot
+    return read_snapshot(prefix, it, o, device)
